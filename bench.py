@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU)
     python bench.py --impl reference --steps K --warmup W    # the reference-style CPU path (oracle) on the host cores
     python bench.py --config c2|c3|c4|c5 ...                 # the other BASELINE.json configs (same JSON shape)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results as DIR/<name>.npy
 
 One "step" = one pass of the hot path over one batch of synthetic closed tracks resident in HBM:
 calc_splines -> assemble banded QP -> interior-point solve -> curvature check -> create_raceline + heading/curvature
@@ -37,6 +38,7 @@ STEP_INTERP = 2.0
 ALG_BYTES_PER_POINT_K2 = 40.0      # SURVEY.md 8d: 32 B reftrack row in + 8 B alpha out
 ALG_BYTES_PER_POINT_SP = 56.0      # shortest path: 32 B reftrack row + 16 B normal in, 8 B alpha out
 IPM_SOURCE = os.path.join(ROOT, "global_racetrajectory_optimization_b200", "csrc", "mincurv_ipm.cu")
+DUMP_LIMIT_BYTES = 64 * 10**6      # --dump-outputs: all files together
 
 # BASELINE.json configs (configs[0] is the reference's own CPU run; c1 is the headline workload of the metric)
 CONFIGS = {
@@ -132,6 +134,23 @@ def measured_traffic():
         return float(prof["dram_bytes_per_qp"]), prof.get("source", "")
     except Exception as e:
         return None, f"no traffic capture ({type(e).__name__})"
+
+
+def dump_outputs(res: dict, out_dir: str, limit: int = DUMP_LIMIT_BYTES, seed: int = 0) -> None:
+    """Writes the results of one step (what a caller of the path receives) as out_dir/<name>.npy in float64; integer
+    results such as status and point counts convert exactly.  If the arrays together exceed `limit` bytes, each keeps the
+    same fraction of its rows (instances), rows = np.sort(np.random.default_rng(seed).choice(len(a), k, replace=False)):
+    the sample depends on the shapes only, and arrays of the same batch size keep the same instances, so the files of two
+    builds run with the same arguments can be compared one to one."""
+    arrs = {k: np.asarray(v.cpu() if hasattr(v, "cpu") else v, dtype=np.float64) for k, v in res.items()}
+    budget = limit - 4096 * len(arrs)                    # (room for the .npy headers)
+    total = sum(a.nbytes for a in arrs.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrs.items():
+        if total > budget and a.ndim > 0:
+            k = a.shape[0] * budget // total
+            a = a[np.sort(np.random.default_rng(seed).choice(a.shape[0], k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class _Timer:
@@ -453,6 +472,8 @@ def run_b200(args) -> dict:
     if rank == 0 and world == 1 and not args.no_cpu_baseline and cfg == "c1":
         line["cpu_baseline"] = cpu_baseline_dense(n, budget_s=25.0)
         line["cpu_baseline_banded"] = cpu_baseline_banded(n, budget_s=15.0)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(res, args.dump_outputs)             # the last timed step's results, written after every measurement
     if world > 1:
         dist.destroy_process_group()
     return line if rank == 0 else None
@@ -665,11 +686,11 @@ def _oracle_worker(job):
         return _oracle_one(rt)
 
 
-def _dense_pool_run(n: int, budget_s: float, max_steps: int = 1000):
+def _dense_pool_run(n: int, budget_s: float = None, steps: int = None):
     """THE protocol of the dense CPU arm (used by cpu_baseline of the b200 line and by --impl reference alike): `workers`
     processes solve different QPs of the workload at the same time, each with cores/workers BLAS threads (a single dense
     solve does not scale past ~8 threads: the 4N x 4N inverse is the only threaded part); one step = `workers` QPs in
-    flight; as many steps as fit the time budget after one warm-up step."""
+    flight; `steps` steps, or as many as fit the time budget, after one warm-up step."""
     import multiprocessing as mp
     from oracle import quadprog_gi
     quadprog_gi.build()
@@ -685,14 +706,17 @@ def _dense_pool_run(n: int, budget_s: float, max_steps: int = 1000):
         t0 = time.perf_counter()
         pool.map(_oracle_worker, jobs)                   # warm-up step (also sizes the run)
         t_first = time.perf_counter() - t0
-        steps = max(1, min(max_steps, int(budget_s / max(t_first, 1e-3)) - 1))
+        bounded = steps is None
+        if bounded:
+            steps = max(1, min(1000, int(budget_s / max(t_first, 1e-3)) - 1))
         t0 = time.perf_counter()
         for _ in range(steps):
             pool.map(_oracle_worker, jobs)
         secs = time.perf_counter() - t0
     sample = (f"each step = {workers} QPs of the workload (N={n}) solved concurrently by {workers} processes x {blas_threads} BLAS "
               f"threads through the dense numpy/LAPACK tph restatement (oracle/tph_dense.py) + Goldfarb-Idnani C solver "
-              f"(oracle/quadprog_gi.c); {steps} steps timed after 1 warm-up step (run bounded to ~{budget_s:.0f} s)")
+              f"(oracle/quadprog_gi.c); {steps} steps timed after 1 warm-up step" +
+              (f" (run bounded to ~{budget_s:.0f} s)" if bounded else ""))
     return steps * workers / secs, cores, workers, steps, secs, sample
 
 
@@ -743,12 +767,12 @@ def cpu_baseline_banded(n: int, budget_s: float = 15.0) -> dict:
 
 def run_reference(args) -> dict:
     """Reference arm: the reference-style CPU path (dense numpy/LAPACK tph restatement + Goldfarb-Idnani in C) on ALL host
-    cores, with the protocol of _dense_pool_run; the run is bounded to a few minutes."""
+    cores, with the protocol of _dense_pool_run; --steps timed steps."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return None
     n = args.npoints or N_POINTS
-    qps, cores, workers, steps, secs, sample = _dense_pool_run(n, 240.0, max_steps=max(1, args.steps))
+    qps, cores, workers, steps, secs, sample = _dense_pool_run(n, steps=args.steps)
     return {"impl": "reference", "metric": METRIC, "value": qps, "unit": UNIT, "n_gpus": int(os.environ.get("WORLD_SIZE", "1")),
             "steps": steps, "warmup": 1, "ms_per_step": 1e3 * secs / steps, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic",
@@ -768,14 +792,21 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="QP instances per GPU (default: the config's)")
     ap.add_argument("--npoints", type=int, default=None, help="points per track (default: the config's)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's results as DIR/<name>.npy (float64, rank 0, at most 64 MB: a fixed, "
+                         "seeded sample of the instances when they do not fit)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 path")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         line = run_reference(args)
     else:
         world = int(os.environ.get("WORLD_SIZE", "1"))
         if args.gpus > 1 and world == 1:
-            # convenience: re-launch ourselves under torchrun (the driver launches torchrun itself)
+            # convenience: re-launch ourselves under torchrun (a launcher that starts torchrun itself sets WORLD_SIZE)
             cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",
                    "--master-addr", "127.0.0.1", "--master-port", "29511", os.path.abspath(__file__), "--gpus", str(args.gpus),
                    "--steps", str(args.steps), "--warmup", str(args.warmup), "--config", args.config]
@@ -783,6 +814,8 @@ def main():
                 cmd += ["--batch", str(args.batch)]
             if args.npoints:
                 cmd += ["--npoints", str(args.npoints)]
+            if args.dump_outputs:
+                cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)]
             sys.exit(subprocess.call(cmd))
         line = run_b200(args)
     if line is not None:

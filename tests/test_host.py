@@ -163,20 +163,15 @@ def test_synthetic_tracks_are_deterministic_and_well_posed():
 
 
 def test_default_pars_are_the_stock_racecar_ini_values():
-    """globaltraj.default_pars() against /root/reference/params/racecar.ini, parsed the way main_globaltraj.py:160-183 does
-    (configparser + json); only in the build container (the GPU box has no /root/reference)."""
-    import configparser
+    """globaltraj.default_pars() against the reference's params/racecar.ini, parsed the way main_globaltraj.py:160-183 does
+    (configparser + json) and stored as tests/golden/racecar_pars.json by tools/make_golden_ref.py."""
     import json
-    import os
-    ini = "/root/reference/params/racecar.ini"
-    if not os.path.exists(ini):
-        pytest.skip("reference tree not present")
     from global_racetrajectory_optimization_b200 import globaltraj
-    parser = configparser.ConfigParser()
-    assert parser.read(ini)
-    ref = {k: json.loads(parser.get("GENERAL_OPTIONS", k)) for k in ("stepsize_opts", "veh_params", "vel_calc_opts")}
-    ref["optim_opts"] = json.loads(parser.get("OPTIMIZATION_OPTIONS", "optim_opts_mincurv"))
-    assert json.loads(parser.get("OPTIMIZATION_OPTIONS", "optim_opts_shortest_path"))["width_opt"] == ref["optim_opts"]["width_opt"]
+    with open(os.path.join(ROOT, "tests", "golden", "racecar_pars.json")) as f:
+        ini = json.load(f)
+    ref = {k: ini["GENERAL_OPTIONS"][k] for k in ("stepsize_opts", "veh_params", "vel_calc_opts")}
+    ref["optim_opts"] = ini["OPTIMIZATION_OPTIONS"]["optim_opts_mincurv"]
+    assert ini["OPTIMIZATION_OPTIONS"]["optim_opts_shortest_path"]["width_opt"] == ref["optim_opts"]["width_opt"]
     mine = globaltraj.default_pars()
     for section, values in mine.items():
         for key, val in values.items():

@@ -7,6 +7,7 @@
     /root/reference/helper_funcs_glob/src/export_traj_ltpl.py      export_traj_ltpl
     /root/reference/helper_funcs_glob/src/import_track.py          import_track
 
+and tests/golden/racecar_pars.json from the reference's params/racecar.ini (write_default_pars), all
 imported from /root/reference in the build container -- so, unlike the tph-based rows, the fixtures of this row are
 PINNED to the reference's own code.  The package's __init__ also imports prep_track / result_plots, which need
 trajectory_planning_helpers and matplotlib (absent offline); both are stubbed with empty modules -- none of the functions
@@ -47,7 +48,23 @@ def load_reference_helpers():
     return helper_funcs_glob
 
 
+def write_default_pars():
+    """tests/golden/racecar_pars.json: the options of params/racecar.ini that globaltraj.default_pars() restates, parsed the
+    way main_globaltraj.py:160-183 parses them (configparser, then json.loads of each value)."""
+    import configparser
+    import json
+    parser = configparser.ConfigParser()
+    assert parser.read(os.path.join(REF, "params", "racecar.ini"))
+    keys = {"GENERAL_OPTIONS": ("stepsize_opts", "veh_params", "vel_calc_opts"),
+            "OPTIMIZATION_OPTIONS": ("optim_opts_shortest_path", "optim_opts_mincurv")}
+    pars = {sec: {k: json.loads(parser.get(sec, k)) for k in ks} for sec, ks in keys.items()}
+    with open(os.path.join(GOLD, "racecar_pars.json"), "w") as f:
+        json.dump(pars, f, indent=1)
+        f.write("\n")
+
+
 def main():
+    write_default_pars()
     hf = load_reference_helpers()
     from oracle import tph_velprofile as VP
     ggv_file = os.path.join(REF, "inputs", "veh_dyn_info", "ggv.csv")
